@@ -60,7 +60,33 @@ def parse_args():
     ap.add_argument("--gather", choices=["peer", "nccl"], default="peer",
                     help="several ranks: how the values reach rank 0 — peer (each rank's epilogue stores into rank 0's HBM through a CUDA IPC mapping) or nccl (gather collective)")
     ap.add_argument("--error-model", default=None, help="haplotype penalty arrays from the reference's error models (reset()), e.g. PCR-free.HiSeq-2500, instead of i.i.d. draws")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the ln-likelihood matrices of the last timed step (rank 0's) to DIR/<name>.npy, "
+                         "float64; above %d MB in all, a seeded sample of each matrix's columns (indices in <name>_columns.npy)" % (DUMP_BYTES // 10**6))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(dirname, outputs):
+    """outputs: [(name, [H, R] float64 tensor)]. Every matrix whole, or, when they would take more than DUMP_BYTES together, the
+    same seeded sample of columns (reads) of each in every run with the same arguments, so that two builds compare value for value."""
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    budget = (DUMP_BYTES - (1 << 20)) // len(outputs)                 # 1 MB for the .npy headers
+    sample = sum(t.numel() for _, t in outputs) * 8 > DUMP_BYTES - (1 << 20)
+    for name, t in outputs:
+        H, R = t.shape
+        if sample:
+            k = max(1, min(R, budget // (8 * (H + 1))))
+            cols = np.sort(np.random.default_rng(0).choice(R, k, replace=False))
+            np.save(os.path.join(dirname, name + "_columns.npy"), cols.astype(np.float64))
+            t = t[:, torch.as_tensor(cols, device=t.device)]
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy().astype(np.float64, copy=False))
 
 
 METRIC = "pair-HMM GCUPS (DP cell-updates/s)"
@@ -380,7 +406,19 @@ def main():
     recv = None
     if world > 1 and rank == 0 and not strong and peer_ring is None:
         recv = [[torch.empty_like(d_out[0]) for _ in range(world)] for _ in range(n_buf)]
-    state = {"k": 0, "gather_ms": [], "launches": 0}
+    state = {"k": 0, "gather_ms": [], "launches": 0, "keep": None}
+
+    def keep(out, reused=False):
+        """--dump-outputs: hold what the last timed step returned. A buffer that a later region of the step writes again is
+        copied first, and the engine's stream waits for the copy."""
+        if state["keep"] is None:
+            return
+        if reused:
+            out = out.clone()
+            ev = torch.cuda.Event()
+            ev.record()
+            eng.wait_event(ev)
+        state["keep"].append(out)
 
     def one_region(dh, dr):
         k = state["k"]
@@ -394,6 +432,7 @@ def main():
             else:
                 out = peer_ring.window(k, rank * max_region_bytes, dh.n, dr.n)
             eng.populate(model_cfg, dh, dr, flank_state=flank_state, out=out)
+            keep(out, reused=len(d_regions) > 1)
             dp = eng.last_dp_kernel_ms()
             state["launches"] += eng.launch_count()
             g0 = torch.cuda.Event(enable_timing=True)
@@ -405,6 +444,7 @@ def main():
             eng.wait_event(gather_done[b])
         out = d_out[b] if (dh.n, dr.n) == (H, R) else None
         out = eng.populate(model_cfg, dh, dr, flank_state=flank_state, out=out)
+        keep(out, reused=len(d_regions) > 1)
         dp = eng.last_dp_kernel_ms()
         state["launches"] += eng.launch_count()
         if world > 1:
@@ -428,9 +468,11 @@ def main():
 
     def step():
         if batched is not None:
-            eng.populate_regions(model_cfg, batched[0], batched[1], batched[2], batched[3],
-                                 flank_states=[flank_state] * len(regions) if flank_state else None, out=flat_out)
+            _, off = eng.populate_regions(model_cfg, batched[0], batched[1], batched[2], batched[3],
+                                          flank_states=[flank_state] * len(regions) if flank_state else None, out=flat_out)
             state["launches"] += eng.launch_count()
+            for m in PairHMMEngine.split_regions(flat_out, off, batched[2], batched[3]):
+                keep(m)
             return eng.last_dp_kernel_ms()
         return sum(one_region(dh, dr) for dh, dr in d_regions)
 
@@ -452,7 +494,9 @@ def main():
     state["launches"] = 0
     sync_all()
     ev0.record()
-    for _ in range(args.steps):
+    for i in range(args.steps):
+        if args.dump_outputs and rank == 0 and i == args.steps - 1:
+            state["keep"] = []
         dp_ms.append(step())
     ev1.record()
     launches = state["launches"]
@@ -463,6 +507,9 @@ def main():
     total_ms = float(ms.item())
     gather_ms = float(np.mean([a.elapsed_time(b) for a, b in state["gather_ms"]])) if state["gather_ms"] else 0.0
     clocks = sampler.stop() if rank == 0 else None
+    kept, state["keep"] = state["keep"], None
+    if kept:
+        dump_outputs(args.dump_outputs, [("likelihoods" if len(kept) == 1 else "likelihoods_region%04d" % g, t) for g, t in enumerate(kept)])
 
     # Did every rank's values land on rank 0? Each rank recomputes its last region locally; rank 0 compares an order-independent bit
     # digest (int64 sum of the float64 bit patterns) of every rank's window of the last slot with that rank's own digest.

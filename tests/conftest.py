@@ -15,22 +15,22 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def coracle():
     from oracle.oracle import COracle, build
-    build(ref=os.path.isdir("/root/reference"))
+    build(ref=False)
     return COracle()
 
 
-@pytest.fixture(scope="session")
-def refkernels():
-    """All reference-kernel ISA builds this host can run ({} where oracle/_ref was never built)."""
-    from oracle.oracle import RefKernel, available_ref_isas
-    return {isa: RefKernel(isa) for isa in available_ref_isas()}
+@pytest.fixture
+def refkernels(request):
+    """The original SIMD kernel, one per instruction-set build ({isa: RefKernel}), replayed from tests/golden (reference_calls.py)."""
+    from reference_calls import reference
+    return reference(request, "kernels")
 
 
-@pytest.fixture(scope="session")
-def refhmm(coracle):
-    """The reference's own hmm::evaluate / hmm::align / PairHMMWrapper (oracle/_ref/libref_hmm.so), or None where it was never built."""
-    from oracle.oracle import RefHMM
-    return RefHMM() if RefHMM.available() else None
+@pytest.fixture
+def refhmm(request):
+    """The original hmm::evaluate / hmm::align / PairHMMWrapper / HaplotypeLikelihoodArray (RefHMM), replayed from tests/golden."""
+    from reference_calls import reference
+    return reference(request, "hmm")
 
 
 @pytest.fixture(scope="session")

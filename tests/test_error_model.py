@@ -1,6 +1,6 @@
 """HaplotypeLikelihoodModel::reset (SURVEY.md a11 / N2): the engine's own error models (octopus_b200/csrc/phmm_error_model.cpp, host C++
-inside libphmm_b200.so) against the UNMODIFIED reference models + lib/tandem compiled from /root/reference (oracle/_ref/libref_errmodel.so),
-array for array — and against committed golden fixtures where the reference build is absent."""
+inside libphmm_b200.so) against the UNMODIFIED reference models + lib/tandem (oracle/_ref/libref_errmodel.so, its answers replayed from
+tests/golden/reference_calls.json.xz), array for array — and against the committed golden fixture of error_model_golden.json."""
 import json
 import os
 
@@ -29,14 +29,11 @@ def repeat_rich_sequence(rng, max_len=400):
     return s[:max_len + 200]
 
 
-@pytest.fixture(scope="module")
-def ref():
-    from oracle.oracle import RefErrorModel, build
-    if os.path.isdir("/root/reference"):
-        build(ref=True)
-    if not RefErrorModel.available():
-        pytest.skip("oracle/_ref/libref_errmodel.so not built (needs /root/reference)")
-    return RefErrorModel()
+@pytest.fixture
+def ref(request):
+    """The original error models + lib/tandem (RefErrorModel), replayed from tests/golden (reference_calls.py)."""
+    from reference_calls import reference
+    return reference(request, "errmodel")
 
 
 def test_tandem_repeat_finder_equals_lib_tandem(ref):
@@ -46,11 +43,11 @@ def test_tandem_repeat_finder_equals_lib_tandem(ref):
     for _ in range(1500):
         s = repeat_rich_sequence(rng)
         for lo, hi in ((1, 5), (1, 3), (1, 2), (2, 3), (1, 1), (2, 2), (3, 3), (1, 4), (2, 5), (1, 8)):
-            assert np.array_equal(m.tandem_repeats(bytes(s), lo, hi), ref.tandem_repeats(s, lo, hi)), (bytes(s), lo, hi)
+            assert ref.tandem_repeats(s, lo, hi) == m.tandem_repeats(bytes(s), lo, hi), (bytes(s), lo, hi)
     # edge cases: empty / single base / string shorter than the period / all one letter / min_period 0
     for s in (b"", b"A", b"AC", b"AAAAAAAAAA", b"ACACACACAC", b"ACGACGACGACG", b"NNNNNN"):
         for lo, hi in ((1, 5), (1, 3), (0, 5), (3, 3), (4, 9)):
-            assert np.array_equal(m.tandem_repeats(s, lo, hi), ref.tandem_repeats(s, lo, hi)), (s, lo, hi)
+            assert ref.tandem_repeats(s, lo, hi) == m.tandem_repeats(s, lo, hi), (s, lo, hi)
 
 
 def test_every_builtin_model_equals_the_reference(ref):
@@ -63,16 +60,15 @@ def test_every_builtin_model_equals_the_reference(ref):
         use_sub = rng.random() < 0.5
         block = m.reset(seqs, is_substitution=subs if use_sub else None, n_threads=3)
         for h, s in enumerate(seqs):
-            want = ref.reset(s, label, subs[h] if use_sub else None)
-            assert want["rc"] >= 0, label
+            rc, want = ref.reset(s, label, subs[h] if use_sub else None)
+            assert rc >= 0, label
             got = block.hap(h)
-            for f in FIELDS:
-                assert np.array_equal(got[f].view(np.uint8), want[f].view(np.uint8)), (label, f, bytes(s))
+            assert want == {f: got[f] for f in FIELDS}, (label, bytes(s))
     for bad in ("PCR-free.HiSeq-9000", "nonsense", "10X.PacBio"):
         from octopus_b200 import PhmmError
         with pytest.raises(PhmmError):
             ErrorModel(bad)
-        assert ref.reset(b"ACGT", bad)["rc"] < 0
+        assert ref.reset(b"ACGT", bad)[0] < 0
 
 
 def test_short_read_models_never_make_an_extension_dearer_than_the_opening():
@@ -110,15 +106,14 @@ def test_custom_model_text_equals_the_reference(ref):
         m = ErrorModel(custom_model_text=text)
         for _ in range(20):
             s = repeat_rich_sequence(rng, 250)
-            want = ref.reset(s, custom_model_text=text)
-            assert want["rc"] == 1
+            rc, want = ref.reset(s, custom_model_text=text)
+            assert rc == 1
             got = m.reset([s]).hap(0)
-            for f in FIELDS:
-                assert np.array_equal(got[f].view(np.uint8), want[f].view(np.uint8)), (f, text, bytes(s))
+            assert want == {f: got[f] for f in FIELDS}, (text, bytes(s))
     for bad in ("A+:3,4\n", "A:\n", ":3\n", "A:3,x\n", "AC 3,4\n"):
         with pytest.raises(PhmmError):
             ErrorModel(custom_model_text=bad)
-        assert ref.reset(b"ACGT", custom_model_text=bad)["rc"] < 0, bad
+        assert ref.reset(b"ACGT", custom_model_text=bad)[0] < 0, bad
 
 
 def test_golden_fixture():

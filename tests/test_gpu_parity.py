@@ -64,8 +64,6 @@ def test_align_scores_match_oracle(engine, coracle, band):
 
 
 def test_align_scores_match_reference_kernel(engine, refkernels):
-    if not refkernels:
-        pytest.skip("oracle/_ref not present")
     from octopus_b200 import synth
     haps, reads, band = synth.make_batch("C2", n_reads=600, n_haps=16)
     rng = np.random.default_rng(9)
@@ -351,8 +349,6 @@ def test_populate_matches_the_compiled_reference_populate(engine, refhmm):
     /root/reference in the authoring container, oracle/_ref/libref_hmm.so) — no restatement in between: same haplotypes, reads,
     flank state and configuration in, the same [H][R] ln-likelihoods out (integer penalties identical; the double epilogue to 1e-4
     relative, in practice a few ulp)."""
-    if refhmm is None:
-        pytest.skip("oracle/_ref/libref_hmm.so not built")
     from octopus_b200 import HaplotypeLikelihoodModel, synth
     rng = np.random.default_rng(8086)
     for trial in range(8):

@@ -346,8 +346,6 @@ def test_align_reads_register_traceback_and_fallbacks(engine, coracle):
 def test_align_pairs_equals_the_mutation_model_hmm(engine, refhmm):
     """N4: phmm_align_pairs on (target haplotype, padded given haplotype) pairs == hmm::PairHMM<VariableGapExtendMutationModel, 32, int>::align,
     the call DeNovoModel makes (denovo_model.cpp:249-262): no SNV mask, scalar mismatch penalty, band 32, offset = band."""
-    if refhmm is None:
-        pytest.skip("oracle/_ref/libref_hmm.so not present")
     from octopus_b200 import HaplotypeLikelihoodModel
     from octopus_b200.batch import pack_haplotypes, pack_reads
     rng = np.random.default_rng(101)
