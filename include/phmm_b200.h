@@ -221,11 +221,34 @@ typedef struct {
 } phmm_regions;
 
 /* out / status (optional): the regions' row-major [H_g][R_g] matrices back to back, region g starting at sum_{g' < g} H_g' * R_g'.
- * Candidate positions come from the device k-mer mapper (config.map_positions) or are the original position only; explicit position
- * lists and templates are not supported here. Errors and statuses as phmm_populate. At most 65535 haplotypes per call. */
+ * Candidate positions come from the device k-mer mapper (config.map_positions) or are the original position only. Errors and statuses
+ * as phmm_populate. At most 65535 haplotypes per call. This is phmm_populate_regions_ex(e, cfg, haps, reads, regions, NULL, NULL, out,
+ * status, space); that call adds paired-read templates and explicit candidate positions. */
 int phmm_populate_regions(phmm_engine* e, const phmm_config* cfg,
                           const phmm_haplotypes* haps, const phmm_reads* reads, const phmm_regions* regions,
                           double* out, int32_t* status, int space);
+
+/* Templates of a many-regions call. Region g owns the templates [template_first[g], template_first[g+1]).
+ * Template t owns the reads [template_off[t], template_off[t+1]); each region's templates cover exactly its reads. */
+typedef struct {
+    const int32_t* template_first;   /* [regions->n + 1], HOST memory whatever `space` says (like the region arrays) */
+    const int64_t* template_off;     /* [template_first[n] + 1], in `space` */
+} phmm_region_templates;
+
+/* Many regions in one call with Octopus's default read linkage: populate(TemplateMap) per region (haplotype_likelihood_array.cpp:105-199,
+ * caller.cpp:465-468) — the value of a template is the sum of its reads' values, in read order (haplotype_likelihood_model.cpp:306-320).
+ *   templates  NULL: one value per read, as phmm_populate_regions. Otherwise out holds the regions' [H_g][T_g] matrices back to back.
+ *              A sample of a multi-sample region is a column range: put the samples' templates back to back.
+ *   positions  NULL: device mapper / original position, as phmm_populate_regions. Otherwise a CSR over the per-read result slots
+ *              (off[sum_g H_g * R_g + 1], the [H_g][R_g] layout of status), validated as in phmm_populate (<= 4096 per pair).
+ *   status     optional, always per read: the regions' [H_g][R_g] matrices back to back.
+ * Template offsets in host memory are checked on the host, device ones on the device; either way a malformed list (not non-decreasing,
+ * or a region's templates not covering exactly its reads) returns PHMM_ERR_INVALID. A short haplotype in one region returns
+ * PHMM_ERR_SHORT_HAPLOTYPE with the statuses and values of every region complete (the caller skips that region, caller.cpp:1182-1188). */
+int phmm_populate_regions_ex(phmm_engine* e, const phmm_config* cfg,
+                             const phmm_haplotypes* haps, const phmm_reads* reads, const phmm_regions* regions,
+                             const phmm_region_templates* templates, const phmm_positions* positions,
+                             double* out, int32_t* status, int space);
 
 /* phmm_populate with device-resident inputs and an output row stride: out[h * out_ld + r], out_ld >= R (status, optional, stays dense
  * [H][R]). `out` is any device-accessible address — in particular a window of ANOTHER GPU's matrix mapped with phmm_ipc_open: the
@@ -250,7 +273,7 @@ int phmm_ipc_close(void* dev_ptr);
 /* Paired / linked reads: HaplotypeLikelihoodArray::populate(TemplateMap) (haplotype_likelihood_array.cpp:105-199). Template t owns
  * the reads [template_off[t], template_off[t+1]) and its value is the sum of its reads' values
  * (HaplotypeLikelihoodModel::evaluate(AlignedTemplate), haplotype_likelihood_model.cpp:306-320). out is [H][n_templates];
- * status (optional) stays per read, [H][R]. Everything else as phmm_populate. */
+ * status (optional) stays per read, [H][R]. Everything else as phmm_populate. The one-region case of phmm_populate_regions_ex. */
 int phmm_populate_templates(phmm_engine* e, const phmm_config* cfg,
                             const phmm_haplotypes* haps, const phmm_reads* reads,
                             const int64_t* template_off, int32_t n_templates,

@@ -9,7 +9,7 @@ PHMM_OK, PHMM_ERR_INVALID, PHMM_ERR_CUDA, PHMM_ERR_BAND, PHMM_ERR_SHORT_HAPLOTYP
 SPACE_HOST, SPACE_DEVICE = 0, 1
 
 EXPORTS = ["phmm_version", "phmm_default_config", "phmm_create", "phmm_destroy", "phmm_last_error", "phmm_launch_count",
-           "phmm_last_dp_kernel_ms", "phmm_last_dp_cells", "phmm_align_scores", "phmm_align_traceback", "phmm_align_reads", "phmm_align_pairs", "phmm_genotype_likelihoods", "phmm_populate", "phmm_populate_templates", "phmm_populate_regions",
+           "phmm_last_dp_kernel_ms", "phmm_last_dp_cells", "phmm_align_scores", "phmm_align_traceback", "phmm_align_reads", "phmm_align_pairs", "phmm_genotype_likelihoods", "phmm_populate", "phmm_populate_templates", "phmm_populate_regions", "phmm_populate_regions_ex",
            "phmm_error_model_create", "phmm_error_model_create_custom", "phmm_error_model_destroy", "phmm_error_model_last_error",
            "phmm_reset_haplotypes", "phmm_tandem_repeats", "phmm_wait_event", "phmm_engine_stream", "phmm_reserve_sms", "phmm_host_alloc", "phmm_host_free",
            "phmm_populate_ld", "phmm_device_alloc", "phmm_device_free", "phmm_ipc_export", "phmm_ipc_open", "phmm_ipc_close"]
@@ -43,6 +43,10 @@ class FlankState(C.Structure):
 
 class Regions(C.Structure):
     _fields_ = [("n", C.c_int32), ("hap_first", C.c_void_p), ("read_first", C.c_void_p), ("flank", C.c_void_p)]
+
+
+class RegionTemplates(C.Structure):
+    _fields_ = [("template_first", C.c_void_p), ("template_off", C.c_void_p)]
 
 
 _lib = None
@@ -94,6 +98,9 @@ def load():
     lib.phmm_populate_regions.restype = C.c_int
     lib.phmm_populate_regions.argtypes = [C.c_void_p, C.POINTER(Config), C.POINTER(Haplotypes), C.POINTER(Reads), C.POINTER(Regions),
                                           C.c_void_p, C.c_void_p, C.c_int]
+    lib.phmm_populate_regions_ex.restype = C.c_int
+    lib.phmm_populate_regions_ex.argtypes = [C.c_void_p, C.POINTER(Config), C.POINTER(Haplotypes), C.POINTER(Reads), C.POINTER(Regions),
+                                             C.POINTER(RegionTemplates), C.POINTER(Positions), C.c_void_p, C.c_void_p, C.c_int]
     lib.phmm_populate_templates.restype = C.c_int
     lib.phmm_populate_templates.argtypes = [C.c_void_p, C.POINTER(Config), C.POINTER(Haplotypes), C.POINTER(Reads), C.c_void_p, C.c_int32,
                                             C.POINTER(Positions), C.POINTER(FlankState), C.c_void_p, C.c_void_p, C.c_int]

@@ -223,33 +223,59 @@ class PairHMMEngine:
         return out
 
     # -- batch boundary ----------------------------------------------------------------------------------------
-    def populate_templates(self, config, haps: HaplotypeBlock, reads: ReadBlock, template_off, flank_state=None):
+    def populate_templates(self, config, haps: HaplotypeBlock, reads: ReadBlock, template_off, flank_state=None, positions=None):
         """HaplotypeLikelihoodArray::populate(TemplateMap): host blocks; template t = reads [template_off[t], template_off[t+1]).
-        Returns the (H, T) matrix: each entry the sum of the template's reads' ln-likelihoods."""
+        Returns the (H, T) matrix: each entry the sum of the template's reads' ln-likelihoods. positions: as in ``populate``."""
         assert not haps.on_device and not reads.on_device
         toff = np.ascontiguousarray(template_off, dtype=np.int64)
         T = len(toff) - 1
         hs, rs, cfg = haps.c_struct(), reads.c_struct(), config.c_struct()
         fstruct = None if flank_state is None else _lib.FlankState(1, int(flank_state[0]), int(flank_state[1]))
+        pstruct, keep = None, None
+        if positions is not None:
+            keep = (np.ascontiguousarray(positions[0], dtype=np.int64), np.ascontiguousarray(positions[1], dtype=np.int32))
+            pstruct = _lib.Positions(keep[0].ctypes.data, keep[1].ctypes.data)
         out = np.empty((haps.n, T), dtype=np.float64)
-        rc = self._lib.phmm_populate_templates(self._h, C.byref(cfg), C.byref(hs), C.byref(rs), toff.ctypes.data, T, None,
+        rc = self._lib.phmm_populate_templates(self._h, C.byref(cfg), C.byref(hs), C.byref(rs), toff.ctypes.data, T,
+                                               C.byref(pstruct) if pstruct is not None else None,
                                                C.byref(fstruct) if fstruct is not None else None, out.ctypes.data, None, _lib.SPACE_HOST)
         if rc != _lib.PHMM_OK:
             self._raise(rc)
         return out
 
-    def populate_regions(self, config, haps: HaplotypeBlock, reads: ReadBlock, hap_first, read_first, flank_states=None, out=None, want_status=False):
-        """Many regions in one call (phmm_populate_regions): region g owns haplotypes [hap_first[g], hap_first[g+1]) and reads
-        [read_first[g], read_first[g+1]). Returns the flat result vector (the regions' [H_g, R_g] matrices back to back) and the
-        per-region offsets into it; ``split_regions`` cuts it into matrices. flank_states: None or a list of (lhs, rhs) / None."""
+    def populate_regions(self, config, haps: HaplotypeBlock, reads: ReadBlock, hap_first, read_first, flank_states=None, out=None, want_status=False,
+                         templates=None, positions=None):
+        """Many regions in one call (phmm_populate_regions / phmm_populate_regions_ex): region g owns haplotypes [hap_first[g], hap_first[g+1])
+        and reads [read_first[g], read_first[g+1]). Returns the flat result vector (the regions' [H_g, R_g] matrices back to back) and the
+        per-region offsets into it; ``split_regions`` cuts it into matrices. flank_states: None or a list of (lhs, rhs) / None.
+
+        templates: None, or (template_off, template_first) as ``batch.concat_templates`` returns them — region g owns the templates
+        [template_first[g], template_first[g+1]), template t the reads [template_off[t], template_off[t+1]). The result then holds the
+        regions' [H_g, T_g] matrices of template values (``split_regions(flat, off, hap_first, template_first)``); the status stays per
+        read ([H_g, R_g]: ``split_regions(status, None, hap_first, read_first)``). template_first is host memory in every case.
+        positions: None, or (off, pos), a CSR of candidate positions over the per-read result slots (the status layout)."""
         dev = haps.on_device
         assert dev == reads.on_device
         hf = np.ascontiguousarray(hap_first, dtype=np.int32)
         rf = np.ascontiguousarray(read_first, dtype=np.int32)
         G = len(hf) - 1
-        sizes = (np.diff(hf).astype(np.int64) * np.diff(rf).astype(np.int64))
-        off = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+        tf = None if templates is None else np.ascontiguousarray(templates[1], dtype=np.int32)
+        off = self.region_offsets(hf, rf if tf is None else tf)
         total = int(off[-1])
+        n_status = int(self.region_offsets(hf, rf)[-1])
+        keep = []
+
+        def in_space(a, dtype):
+            if dev:
+                import torch
+                t = a if _is_torch(a) else torch.as_tensor(np.ascontiguousarray(a, dtype=dtype), device=haps.seq.device)
+                keep.append(t)
+                return t.data_ptr()
+            a = np.ascontiguousarray(a, dtype=dtype)
+            keep.append(a)
+            return a.ctypes.data
+        tstruct = None if tf is None else _lib.RegionTemplates(tf.ctypes.data, in_space(templates[0], np.int64))
+        pstruct = None if positions is None else _lib.Positions(in_space(positions[0], np.int64), in_space(positions[1], np.int32))
         fl = None
         if flank_states is not None:
             fl = (_lib.FlankState * G)()
@@ -265,24 +291,38 @@ class PairHMMEngine:
             if out is None:
                 out = torch.empty(total, dtype=torch.float64, device=haps.seq.device)
             if want_status:
-                status = torch.empty(total, dtype=torch.int32, device=haps.seq.device)
+                status = torch.empty(n_status, dtype=torch.int32, device=haps.seq.device)
             op, sp = out.data_ptr(), (status.data_ptr() if want_status else None)
         else:
             if out is None:
                 out = np.empty(total, dtype=np.float64)
             if want_status:
-                status = np.empty(total, dtype=np.int32)
+                status = np.empty(n_status, dtype=np.int32)
             op, sp = out.ctypes.data, (status.ctypes.data if want_status else None)
-        rc = self._lib.phmm_populate_regions(self._h, C.byref(cfg), C.byref(hs), C.byref(rs), C.byref(regs), op, sp,
-                                             _lib.SPACE_DEVICE if dev else _lib.SPACE_HOST)
+        space = _lib.SPACE_DEVICE if dev else _lib.SPACE_HOST
+        if tstruct is None and pstruct is None:
+            rc = self._lib.phmm_populate_regions(self._h, C.byref(cfg), C.byref(hs), C.byref(rs), C.byref(regs), op, sp, space)
+        else:
+            rc = self._lib.phmm_populate_regions_ex(self._h, C.byref(cfg), C.byref(hs), C.byref(rs), C.byref(regs),
+                                                    C.byref(tstruct) if tstruct is not None else None,
+                                                    C.byref(pstruct) if pstruct is not None else None, op, sp, space)
         if rc != _lib.PHMM_OK and not (rc == _lib.PHMM_ERR_SHORT_HAPLOTYPE and want_status):
             self._raise(rc)
         return (out, off, status) if want_status else (out, off)
 
     @staticmethod
-    def split_regions(flat, off, hap_first, read_first):
-        """The per-region [H_g, R_g] views of a populate_regions result."""
-        return [flat[int(off[g]):int(off[g + 1])].reshape(int(hap_first[g + 1] - hap_first[g]), int(read_first[g + 1] - read_first[g]))
+    def region_offsets(hap_first, col_first):
+        """Where each region's [H_g, C_g] matrix starts in a flat populate_regions result (C_g: reads, or templates)."""
+        sizes = np.diff(np.asarray(hap_first, dtype=np.int64)) * np.diff(np.asarray(col_first, dtype=np.int64))
+        return np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+
+    @staticmethod
+    def split_regions(flat, off, hap_first, col_first):
+        """The per-region [H_g, C_g] views of a populate_regions result: col_first is read_first for per-read results (and the status),
+        template_first for template values. off: the offsets populate_regions returned, or None (computed from the widths)."""
+        if off is None:
+            off = PairHMMEngine.region_offsets(hap_first, col_first)
+        return [flat[int(off[g]):int(off[g + 1])].reshape(int(hap_first[g + 1] - hap_first[g]), int(col_first[g + 1] - col_first[g]))
                 for g in range(len(off) - 1)]
 
     def populate(self, config, haps: HaplotypeBlock, reads: ReadBlock, positions=None, flank_state=None, out=None,

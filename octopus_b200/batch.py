@@ -187,3 +187,18 @@ def concat_blocks(hap_blocks, read_blocks):
     hap_first = np.concatenate([[0], np.cumsum([b.n for b in hap_blocks])]).astype(np.int32)
     read_first = np.concatenate([[0], np.cumsum([b.n for b in read_blocks])]).astype(np.int32)
     return haps, reads, hap_first, read_first
+
+
+def concat_templates(per_region_template_offs):
+    """Templates of regions back to back, matching ``concat_blocks``: region g's template_off (local: from 0 to its read count) →
+    (template_off over the concatenated reads, int64; template_first over the regions, int32) — PairHMMEngine.populate_regions'
+    ``templates`` argument."""
+    offs = [np.asarray(o, dtype=np.int64) for o in per_region_template_offs]
+    parts, base = [np.zeros(1, dtype=np.int64)], 0
+    for o in offs:
+        if len(o) < 2 or o[0] != 0 or (np.diff(o) < 0).any():
+            raise ValueError("a region's template offsets must start at 0, be non-decreasing and hold at least one template")
+        parts.append(o[1:] + base)
+        base += int(o[-1])
+    template_first = np.concatenate([[0], np.cumsum([len(o) - 1 for o in offs])]).astype(np.int32)
+    return np.concatenate(parts), template_first

@@ -294,6 +294,19 @@ struct HaplotypeBlock   // what HaplotypeLikelihoodModel::reset derives per hapl
         begin.push_back(mapped_begin);
         off.push_back(static_cast<std::int64_t>(seq.size()));
     }
+    void append(const HaplotypeBlock& other)   // the penalty arrays of both blocks must be filled
+    {
+        const auto base = static_cast<std::int64_t>(seq.size());
+        seq.insert(seq.end(), other.seq.begin(), other.seq.end());
+        snv_mask_fwd.insert(snv_mask_fwd.end(), other.snv_mask_fwd.begin(), other.snv_mask_fwd.end());
+        snv_mask_rev.insert(snv_mask_rev.end(), other.snv_mask_rev.begin(), other.snv_mask_rev.end());
+        snv_prior_fwd.insert(snv_prior_fwd.end(), other.snv_prior_fwd.begin(), other.snv_prior_fwd.end());
+        snv_prior_rev.insert(snv_prior_rev.end(), other.snv_prior_rev.begin(), other.snv_prior_rev.end());
+        gap_open.insert(gap_open.end(), other.gap_open.begin(), other.gap_open.end());
+        gap_extend.insert(gap_extend.end(), other.gap_extend.begin(), other.gap_extend.end());
+        begin.insert(begin.end(), other.begin.begin(), other.begin.end());
+        for (std::size_t i = 1; i < other.off.size(); ++i) off.push_back(base + other.off[i]);
+    }
     std::size_t size() const noexcept { return off.size() - 1; }
     phmm_haplotypes view() const noexcept
     {
@@ -472,6 +485,8 @@ public:
     const double* data() const noexcept { return likelihoods_.data(); }   // [haplotype][all samples' columns], row-major
 
 private:
+    friend class RegionBatch;   // fills arrays from the result of one many-regions call (fill_from)
+
     Engine engine_;
     phmm_config config_;
     pinned_vector<double> likelihoods_;
@@ -481,6 +496,12 @@ private:
     std::size_t num_haplotypes_ = 0;
     mutable std::ptrdiff_t primed_ = -1;
 
+    // samples_ / sample_off_ already set: the [num_haplotypes][total width] values, row-major
+    void fill_from(std::size_t num_haplotypes, const double* values)
+    {
+        num_haplotypes_ = num_haplotypes;
+        likelihoods_.assign(values, values + num_haplotypes * total_width());
+    }
     void begin_samples(std::size_t n) { samples_.clear(); samples_.reserve(n); sample_off_.assign(1, 0); unprime(); }
     void add_sample(const SampleName& name, std::size_t n) { samples_.push_back(name); sample_off_.push_back(sample_off_.back() + n); }
     std::size_t total_width() const noexcept { return sample_off_.back(); }
@@ -521,6 +542,167 @@ private:
             }
         }
         engine_.check(rc);
+    }
+};
+
+// Many independent regions in ONE engine call (phmm_populate_regions_ex): a batch front end for a caller that has several regions
+// ready at once (Octopus's region tasks). Each region is what one HaplotypeLikelihoodArray::populate call takes — a ReadMap or a
+// TemplateMap (the two kinds may be mixed: a ReadMap region then rides along as one-read templates, whose sums are the reads' values
+// exactly), its haplotypes (penalty arrays filled) and an optional flank state. run() yields one array per region, in the order added,
+// with the samples, widths and values populate() gives for that region alone. A region with a short haplotype is reported in its
+// result (as ShortHaplotypeError would report it) and the other regions are filled all the same.
+class RegionBatch
+{
+public:
+    using ReadMap = HaplotypeLikelihoodArray::ReadMap;
+    using TemplateMap = HaplotypeLikelihoodArray::TemplateMap;
+
+    struct Result
+    {
+        HaplotypeLikelihoodArray likelihoods;
+        bool short_haplotype = false;           // populate() would have thrown ShortHaplotypeError {haplotype_index, required_extension}
+        std::size_t haplotype_index = 0;
+        unsigned required_extension = 0;
+        void check() const { if (short_haplotype) throw ShortHaplotypeError {haplotype_index, required_extension}; }
+    };
+
+    explicit RegionBatch(phmm_config config, Engine engine = Engine {}) : config_ {config}, engine_ {std::move(engine)}
+    {
+        if (config.max_indel_error > 256) throw TooLargeBandSizeError {static_cast<unsigned>(config.max_indel_error)};
+    }
+
+    // Each add() copies the region into the batch's page-locked blocks and returns its index.
+    std::size_t add(const ReadMap& reads, const HaplotypeBlock& haplotypes, const FlankState* flank_state = nullptr)
+    {
+        std::size_t n_reads = 0;
+        for (const auto& p : reads) n_reads += p.second.size();
+        Region g = begin_region(haplotypes, n_reads, flank_state, false);
+        for (const auto& p : reads) {
+            g.samples.push_back(p.first); g.widths.push_back(p.second.size());
+            if (g.in_call()) reads_.append(p.second);
+        }
+        regions_.push_back(std::move(g));
+        return regions_.size() - 1;
+    }
+    std::size_t add(const TemplateMap& templates, const HaplotypeBlock& haplotypes, const FlankState* flank_state = nullptr)
+    {
+        for (const auto& p : templates) {
+            const TemplateBlock& tb = p.second;
+            if (tb.off.empty() || tb.off.front() != 0 || static_cast<std::size_t>(tb.off.back()) != tb.reads.size() ||
+                !std::is_sorted(tb.off.begin(), tb.off.end())) throw std::invalid_argument {"RegionBatch: template offsets must cover the sample's reads"};
+        }
+        std::size_t n_reads = 0;
+        for (const auto& p : templates) n_reads += p.second.reads.size();
+        Region g = begin_region(haplotypes, n_reads, flank_state, true);
+        for (const auto& p : templates) {
+            g.samples.push_back(p.first); g.widths.push_back(p.second.size());
+            if (!g.in_call()) continue;
+            const auto base = static_cast<std::int64_t>(reads_.size() - g.read0);
+            for (std::size_t t = 1; t < p.second.off.size(); ++t) g.template_off.push_back(base + p.second.off[t]);
+            reads_.append(p.second.reads);
+        }
+        regions_.push_back(std::move(g));
+        return regions_.size() - 1;
+    }
+    std::size_t size() const noexcept { return regions_.size(); }
+    void clear() { regions_.clear(); haps_ = HaplotypeBlock {}; reads_ = ReadBlock {}; }
+
+    std::vector<Result> run()
+    {
+        std::vector<Result> results;
+        results.reserve(regions_.size());
+        bool any_templates = false;
+        std::vector<std::int32_t> hap_first {0}, read_first {0}, template_first {0};
+        std::vector<phmm_flank_state> flanks;
+        pinned_vector<std::int64_t> template_off {0};
+        std::size_t n_out = 0, n_status = 0;
+        for (const Region& g : regions_) any_templates = any_templates || g.templated;
+        for (const Region& g : regions_) {
+            if (!g.in_call()) continue;
+            hap_first.push_back(static_cast<std::int32_t>(g.hap0 + g.n_haps));
+            read_first.push_back(static_cast<std::int32_t>(g.read0 + g.n_reads));
+            flanks.push_back(g.flank);
+            if (any_templates) {
+                const std::size_t base = g.read0;
+                if (g.templated) for (std::size_t t = 1; t < g.template_off.size(); ++t) template_off.push_back(static_cast<std::int64_t>(base) + g.template_off[t]);
+                else for (std::size_t r = 1; r <= g.n_reads; ++r) template_off.push_back(static_cast<std::int64_t>(base + r));
+                template_first.push_back(static_cast<std::int32_t>(template_off.size() - 1));
+            }
+            n_out += g.n_haps * g.width();
+            n_status += g.n_haps * g.n_reads;
+        }
+        int rc = PHMM_OK;
+        if (flanks.size()) {
+            out_.resize(n_out);
+            status_.resize(n_status);
+            const auto hv = haps_.view();
+            const auto rv = reads_.view();
+            const phmm_regions regions {static_cast<std::int32_t>(flanks.size()), hap_first.data(), read_first.data(), flanks.data()};
+            const phmm_region_templates templates {template_first.data(), template_off.data()};
+            rc = phmm_populate_regions_ex(engine_.get(), &config_, &hv, &rv, &regions, any_templates ? &templates : nullptr, nullptr,
+                                          out_.data(), status_.data(), PHMM_SPACE_HOST);
+            if (rc != PHMM_ERR_SHORT_HAPLOTYPE) engine_.check(rc);
+        }
+        std::size_t out_at = 0, status_at = 0;
+        for (const Region& g : regions_) {
+            Result res {HaplotypeLikelihoodArray {config_, engine_}};
+            HaplotypeLikelihoodArray& a = res.likelihoods;
+            a.begin_samples(g.samples.size());
+            for (std::size_t s = 0; s < g.samples.size(); ++s) a.add_sample(g.samples[s], g.widths[s]);
+            if (!g.in_call()) {
+                const std::vector<double> zeros(g.n_haps * g.width(), 0.0);   // no reads: every template sums to 0
+                a.fill_from(g.n_haps, zeros.data());
+            } else {
+                a.fill_from(g.n_haps, out_.data() + out_at);
+                if (rc == PHMM_ERR_SHORT_HAPLOTYPE) {
+                    for (std::size_t i = 0; i < g.n_haps * g.n_reads; ++i) {
+                        const std::int32_t st = status_[status_at + i];
+                        if ((st & 0xFFFF) == PHMM_STATUS_SHORT_HAP) {
+                            res.short_haplotype = true;
+                            res.haplotype_index = i / g.n_reads;
+                            res.required_extension = static_cast<unsigned>(static_cast<std::uint32_t>(st) >> 16);
+                            break;
+                        }
+                    }
+                }
+                out_at += g.n_haps * g.width();
+                status_at += g.n_haps * g.n_reads;
+            }
+            results.push_back(std::move(res));
+        }
+        return results;
+    }
+
+private:
+    struct Region
+    {
+        std::vector<SampleName> samples;
+        std::vector<std::size_t> widths;
+        std::size_t hap0 = 0, n_haps = 0, read0 = 0, n_reads = 0;
+        bool templated = false;
+        phmm_flank_state flank {0, 0, 0};
+        std::vector<std::int64_t> template_off {0};   // over the region's reads
+        std::size_t width() const { std::size_t w = 0; for (const std::size_t x : widths) w += x; return w; }
+        bool in_call() const { return n_haps > 0 && n_reads > 0; }
+    };
+    phmm_config config_;
+    Engine engine_;
+    HaplotypeBlock haps_;
+    ReadBlock reads_;
+    std::vector<Region> regions_;
+    pinned_vector<double> out_;            // page-locked result buffers kept across runs
+    pinned_vector<std::int32_t> status_;
+
+    // a region without haplotypes or reads stays out of the call and out of the blocks (run() fills its array)
+    Region begin_region(const HaplotypeBlock& haplotypes, std::size_t n_reads, const FlankState* flank_state, bool templated)
+    {
+        Region g;
+        g.templated = templated;
+        if (flank_state) g.flank = phmm_flank_state {1, flank_state->lhs_flank, flank_state->rhs_flank};
+        g.hap0 = haps_.size(); g.n_haps = haplotypes.size();
+        g.read0 = reads_.size(); g.n_reads = n_reads;
+        if (g.in_call()) haps_.append(haplotypes);
+        return g;
     }
 };
 

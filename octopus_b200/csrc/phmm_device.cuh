@@ -48,6 +48,7 @@ constexpr uint32_t kInf16    = 0x7000u;   // +inf of the packed 16-bit lanes; kI
 constexpr uint32_t kInf16x2  = kInf16 | (kInf16 << 16);
 constexpr int      kInf32    = 1 << 28;   // +inf of the int32 kernel
 constexpr int      kFlagOpenBelowExtend = 16;    // engine flag word: some haplotype base has gap_open < gap_extend (see dp_pair, OGE)
+constexpr int      kFlagBadTemplates = 32;       // engine flag word: device-resident template offsets failed k_check_templates
 constexpr int      kMaxScore16 = 0x7000 - 1024;  // a read whose sum of qualities is below this cannot overflow a 16-bit lane
 
 // Read row half-word: code | qual << 8 (code: A0 C1 G2 T3, N4). Reads with an 'N' are served by the 32-bit kernel (its

@@ -65,6 +65,7 @@ struct phmm_engine {
     DBuf tab_f, tab_r, rowhalf, info, flags, best, status, out, slow, counters, pairs, generic_reads, wide_reads, bp, regs, rregion, rpbase, rpstride;
     DBuf tasks_lane, tasks_generic, works, scores;
     DBuf rhash, kbins, kitems, kpos, kcnt, ftasks, fcnt, gtasks, atasks, gcnt, sched, sorted, fb_scratch, fb_pairs, npre_f, npre_r;
+    DBuf toff, tregion;                 // template offsets (host-space calls) and the region of every template
     std::vector<cudaEvent_t> tile_events;
     std::vector<int2> info_host;
     // per-kernel launch configuration already applied / queried (the runtime calls are not free and need not be repeated)
@@ -342,7 +343,8 @@ void phmm_destroy(phmm_engine* e)
                    &e->r_off, &e->r_bases, &e->r_quals, &e->r_mapq, &e->r_rev, &e->r_begin, &e->c_off, &e->c_pos,
                    &e->tab_f, &e->tab_r, &e->rowhalf, &e->info, &e->flags, &e->best, &e->status, &e->out, &e->slow,
                    &e->counters, &e->pairs, &e->generic_reads, &e->wide_reads, &e->bp, &e->regs, &e->rregion, &e->rpbase, &e->rpstride, &e->tasks_lane, &e->tasks_generic, &e->works, &e->scores,
-                   &e->rhash, &e->kbins, &e->kitems, &e->kpos, &e->kcnt, &e->ftasks, &e->fcnt, &e->gtasks, &e->atasks, &e->gcnt, &e->sched, &e->sorted, &e->fb_scratch, &e->fb_pairs, &e->npre_f, &e->npre_r};
+                   &e->rhash, &e->kbins, &e->kitems, &e->kpos, &e->kcnt, &e->ftasks, &e->fcnt, &e->gtasks, &e->atasks, &e->gcnt, &e->sched, &e->sorted, &e->fb_scratch, &e->fb_pairs, &e->npre_f, &e->npre_r,
+                   &e->toff, &e->tregion};
     for (DBuf* b : all) b->release();
     for (cudaEvent_t ev : e->tile_events) cudaEventDestroy(ev);
     if (e->ev0) cudaEventDestroy(e->ev0);
@@ -775,13 +777,16 @@ int phmm_align_pairs(phmm_engine* e, const phmm_config* cfg,
 // One synchronous pass over (all haplotypes) x (the given reads). out / status are written with a row pitch of out_pitch
 // elements (0: dense [H][R]) so that a read chunk can land in its column block of the caller's [H][R_total] matrix.
 // One region list for every call: phmm_populate is the one-region case. Host copies of the region arrays (a few KB).
+// With templates, every region owns at least one template and the template values of the call number total_tout.
 struct RegionSetup {
     std::vector<RegionInfo> regs;
-    long long total_out = 0;
-    int Hmax = 0;
+    long long total_out = 0, total_tout = 0;
+    int Hmax = 0, n_templates = 0;
     bool any_flank = false;
 };
 
+// template_off (CSR over the reads, n_templates + 1 entries, in `space`): one value per (haplotype, template) instead of per read. Host
+// offsets have been validated by the caller; device ones are checked here, on the device.
 static int populate_impl(phmm_engine* e, const phmm_config* cfg,
                          const phmm_haplotypes* haps, const phmm_reads* reads,
                          const phmm_positions* positions, const phmm_flank_state* flank,
@@ -812,9 +817,12 @@ static int populate_impl(phmm_engine* e, const phmm_config* cfg,
         RegionInfo g {};
         g.h0 = 0; g.nH = H_total; g.r0 = 0; g.nR = R; g.out_off = 0;
         g.use_flanks = fl ? 1 : 0; g.lhs = fl ? (int)flank->lhs_flank : 0; g.rhs = fl ? (int)flank->rhs_flank : 0;
+        g.t0 = 0; g.nT = template_off ? n_templates : 0; g.tout_off = 0;
         single.regs.push_back(g); single.total_out = (long long)H_total * R; single.Hmax = H_total; single.any_flank = fl;
+        single.n_templates = g.nT; single.total_tout = (long long)H_total * g.nT;
         multi = &single;
     }
+    const int T = template_off ? multi->n_templates : 0;
     const int G = (int)multi->regs.size();
     // H: haplotype slots per read (the widest region); HR: result slots of the whole call
     const int H = multi->Hmax;
@@ -856,7 +864,6 @@ static int populate_impl(phmm_engine* e, const phmm_config* cfg,
     // candidates a pair can have: listed / mapped positions + the original position + the shifted fallback
     // (haplotype_likelihood_model.cpp:211-259); at most (listed + 1) of them reach a DP
     int max_cand = 2, max_dp_per_pair = 1;
-    if (positions && positions->off && positions->pos && G > 1) { e->err = "candidate position lists are not supported with several regions"; return PHMM_ERR_INVALID; }
     if (positions && positions->off && positions->pos) {
         // Candidate lists: CSR arrays on the device; the host needs the total (to size the copy) and the longest list (to size the
         // per-read task lists: the reference accepts lists of any length) — reduced on the device, 32 bytes back.
@@ -1269,25 +1276,24 @@ static int populate_impl(phmm_engine* e, const phmm_config* cfg,
 
     chunk_order.publish(true);
     lap("tiles enqueued");
-    CU(e->out.ensure((size_t)HR * sizeof(double)));
-    double* d_out = (space == PHMM_SPACE_DEVICE && !template_off) ? out : e->out.as<double>();
-    {
-        const long long threads = (long long)H * R;
-        k_epilogue<<<(unsigned)((threads + 255) / 256), 256, 0, e->stream>>>(p.best, p.status, s.rd, e->regs.as<RegionInfo>(), H, cfg->use_mapping_quality,
-                                                                             cfg->mapping_quality_cap, cfg->mapping_quality_cap_trigger, d_out,
-                                                                             d_out == out && space == PHMM_SPACE_DEVICE && out_pitch > R ? out_pitch - R : 0LL);
-    }
-    LAUNCHED();
-    CU(cudaGetLastError());
-    if (template_off && G > 1) { e->err = "templates are not supported with several regions"; return PHMM_ERR_INVALID; }
     if (template_off) {
-        // paired / linked reads: one value per (haplotype, template)
+        // paired / linked reads: one value per (haplotype, template), summed straight from the integer penalties
         const long long* d_toff;
-        if ((rc = stage(e, e->tasks_lane, (const long long*)template_off, (size_t)n_templates + 1, space, &d_toff))) return rc;
-        const long long HT = (long long)H * n_templates;
-        CU(e->tasks_generic.ensure((size_t)HT * sizeof(double)));
-        double* d_tout = space == PHMM_SPACE_DEVICE ? out : e->tasks_generic.as<double>();
-        k_template_sum<<<(unsigned)((HT + 255) / 256), 256, 0, e->stream>>>(d_out, H, R, d_toff, n_templates, d_tout);
+        if ((rc = stage(e, e->toff, (const long long*)template_off, (size_t)T + 1, space, &d_toff))) return rc;
+        CU(e->tregion.ensure((size_t)T * sizeof(int)));
+        k_template_regions<<<(T + 255) / 256, 256, 0, e->stream>>>(T, G, e->regs.as<RegionInfo>(), e->tregion.as<int>());
+        LAUNCHED();
+        if (space == PHMM_SPACE_DEVICE) {
+            k_check_templates<<<(T + 255) / 256, 256, 0, e->stream>>>(T, d_toff, e->tregion.as<int>(), e->regs.as<RegionInfo>(), e->flags.as<int>());
+            LAUNCHED();
+        }
+        const long long HT = multi->total_tout;
+        CU(e->out.ensure((size_t)std::max<long long>(HT, 1) * sizeof(double)));
+        double* d_tout = space == PHMM_SPACE_DEVICE ? out : e->out.as<double>();
+        const long long threads = (long long)H * T;
+        k_template_epilogue<<<(unsigned)((threads + 255) / 256), 256, 0, e->stream>>>(p.best, p.status, s.rd, e->regs.as<RegionInfo>(), H, T, d_toff,
+                                                                                      e->tregion.as<int>(), cfg->use_mapping_quality, cfg->mapping_quality_cap,
+                                                                                      cfg->mapping_quality_cap_trigger, e->flags.as<int>(), d_tout);
         LAUNCHED();
         CU(cudaGetLastError());
         if (space == PHMM_SPACE_HOST) {
@@ -1296,16 +1302,26 @@ static int populate_impl(phmm_engine* e, const phmm_config* cfg,
         } else if (status) {
             CU(cudaMemcpyAsync(status, p.status, (size_t)HR * sizeof(int), cudaMemcpyDeviceToDevice, e->stream));
         }
-    } else if (space == PHMM_SPACE_HOST) {
-        if (out_pitch == 0 || out_pitch == R) {
-            CU(cudaMemcpyAsync(out, d_out, (size_t)HR * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-            if (status) CU(cudaMemcpyAsync(status, p.status, (size_t)HR * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
-        } else {
-            CU(cudaMemcpy2DAsync(out, (size_t)out_pitch * sizeof(double), d_out, (size_t)R * sizeof(double), (size_t)R * sizeof(double), H, cudaMemcpyDeviceToHost, e->stream));
-            if (status) CU(cudaMemcpy2DAsync(status, (size_t)out_pitch * sizeof(int), p.status, (size_t)R * sizeof(int), (size_t)R * sizeof(int), H, cudaMemcpyDeviceToHost, e->stream));
+    } else {
+        CU(e->out.ensure((size_t)HR * sizeof(double)));
+        double* d_out = space == PHMM_SPACE_DEVICE ? out : e->out.as<double>();
+        const long long threads = (long long)H * R;
+        k_epilogue<<<(unsigned)((threads + 255) / 256), 256, 0, e->stream>>>(p.best, p.status, s.rd, e->regs.as<RegionInfo>(), H, cfg->use_mapping_quality,
+                                                                             cfg->mapping_quality_cap, cfg->mapping_quality_cap_trigger, d_out,
+                                                                             d_out == out && space == PHMM_SPACE_DEVICE && out_pitch > R ? out_pitch - R : 0LL);
+        LAUNCHED();
+        CU(cudaGetLastError());
+        if (space == PHMM_SPACE_HOST) {
+            if (out_pitch == 0 || out_pitch == R) {
+                CU(cudaMemcpyAsync(out, d_out, (size_t)HR * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+                if (status) CU(cudaMemcpyAsync(status, p.status, (size_t)HR * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+            } else {
+                CU(cudaMemcpy2DAsync(out, (size_t)out_pitch * sizeof(double), d_out, (size_t)R * sizeof(double), (size_t)R * sizeof(double), H, cudaMemcpyDeviceToHost, e->stream));
+                if (status) CU(cudaMemcpy2DAsync(status, (size_t)out_pitch * sizeof(int), p.status, (size_t)R * sizeof(int), (size_t)R * sizeof(int), H, cudaMemcpyDeviceToHost, e->stream));
+            }
+        } else if (status) {
+            CU(cudaMemcpyAsync(status, p.status, (size_t)HR * sizeof(int), cudaMemcpyDeviceToDevice, e->stream));
         }
-    } else if (status) {
-        CU(cudaMemcpyAsync(status, p.status, (size_t)HR * sizeof(int), cudaMemcpyDeviceToDevice, e->stream));
     }
     int flags_host[1] = {0};
     lap("enqueued");
@@ -1314,6 +1330,7 @@ static int populate_impl(phmm_engine* e, const phmm_config* cfg,
     CU(cudaStreamSynchronize(e->stream));
     lap("done");
     if (flags_host[0] & 1) { e->err = "snv prior / gap penalty outside [0,127]"; return PHMM_ERR_INVALID; }
+    if (flags_host[0] & kFlagBadTemplates) { e->err = "template offsets must be non-decreasing and cover each region's reads exactly"; return PHMM_ERR_INVALID; }
     if (trace && n_timed) { float ms = 0.f; cudaEventElapsedTime(&ms, e->tile_events[0], e->tile_events[2 * n_timed - 1]); std::fprintf(stderr, "[phmm %p] dp span %.3f ms\n", (void*)e, ms); }
     if (n_timed) {
         double total = 0.0;
@@ -1334,8 +1351,17 @@ int phmm_populate_regions(phmm_engine* e, const phmm_config* cfg,
                           const phmm_haplotypes* haps, const phmm_reads* reads, const phmm_regions* regions,
                           double* out, int32_t* status, int space)
 {
+    return phmm_populate_regions_ex(e, cfg, haps, reads, regions, nullptr, nullptr, out, status, space);
+}
+
+int phmm_populate_regions_ex(phmm_engine* e, const phmm_config* cfg,
+                             const phmm_haplotypes* haps, const phmm_reads* reads, const phmm_regions* regions,
+                             const phmm_region_templates* templates, const phmm_positions* positions,
+                             double* out, int32_t* status, int space)
+{
     if (!e) return PHMM_ERR_INVALID;
     if (!regions || regions->n <= 0 || !regions->hap_first || !regions->read_first || !haps || !reads) { e->err = "null / empty region list"; return PHMM_ERR_INVALID; }
+    if (templates && (!templates->template_first || !templates->template_off)) { e->err = "null template arrays"; return PHMM_ERR_INVALID; }
     RegionSetup setup;
     setup.regs.resize((size_t)regions->n);
     if (regions->hap_first[0] != 0 || regions->read_first[0] != 0 || regions->hap_first[regions->n] != haps->n || regions->read_first[regions->n] != reads->n) {
@@ -1353,7 +1379,28 @@ int phmm_populate_regions(phmm_engine* e, const phmm_config* cfg,
         r.use_flanks = fl ? 1 : 0; r.lhs = fl ? (int)regions->flank[g].lhs_flank : 0; r.rhs = fl ? (int)regions->flank[g].rhs_flank : 0; r.pad = 0;
         setup.any_flank = setup.any_flank || fl;
     }
-    return populate_impl(e, cfg, haps, reads, nullptr, nullptr, out, status, space, 0, nullptr, 0, &setup);
+    if (templates) {
+        const int32_t* tf = templates->template_first;
+        if (tf[0] != 0) { e->err = "template_first must start at 0"; return PHMM_ERR_INVALID; }
+        for (int g = 0; g < regions->n; ++g) {
+            RegionInfo& r = setup.regs[(size_t)g];
+            r.t0 = tf[g]; r.nT = tf[g + 1] - tf[g];
+            // a region has reads, so at least one template covers them
+            if (r.nT <= 0) { e->err = "template_first must be increasing: every region needs at least one template"; return PHMM_ERR_INVALID; }
+            r.tout_off = setup.total_tout;
+            setup.total_tout += (long long)r.nH * r.nT;
+        }
+        setup.n_templates = tf[regions->n];
+        if (space == PHMM_SPACE_HOST) {
+            const int64_t* to = templates->template_off;
+            for (int t = 0; t < setup.n_templates; ++t) if (to[t + 1] < to[t]) { e->err = "template offsets must be non-decreasing"; return PHMM_ERR_INVALID; }
+            for (const RegionInfo& r : setup.regs) {
+                if (to[r.t0] != r.r0 || to[r.t0 + r.nT] != (int64_t)r.r0 + r.nR) { e->err = "each region's templates must cover exactly its reads"; return PHMM_ERR_INVALID; }
+            }
+        }
+    }
+    return populate_impl(e, cfg, haps, reads, positions, nullptr, out, status, space, 0, templates ? templates->template_off : nullptr,
+                         setup.n_templates, &setup);
 }
 
 int phmm_populate_ld(phmm_engine* e, const phmm_config* cfg,

@@ -37,7 +37,8 @@ struct DevReads {
     const long long* pbase;
     const int* pstride;
 };
-struct RegionInfo { int h0, nH, r0, nR; long long out_off; int lhs, rhs, use_flanks, pad; };
+// Templates (phmm_populate_regions_ex): region g owns templates [t0, t0 + nT), its [nH][nT] template values start at tout_off.
+struct RegionInfo { int h0, nH, r0, nR; long long out_off; int lhs, rhs, use_flanks, t0; long long tout_off; int nT, pad; };
 __device__ __forceinline__ long long pair_slot(const DevReads& rd, const int h, const int r) { return rd.pbase[r] + (long long)h * rd.pstride[r]; }
 constexpr int kReadNonACGT  = 1;   // read holds a byte outside ACGT → generic path
 constexpr int kReadUnsafe16 = 2;   // sum of qualities too large for a 16-bit lane, or a quality > 127
@@ -169,6 +170,31 @@ __global__ void k_read_regions(const int n_reads, const int n_regions, const Reg
     region[r] = lo;
     pbase[r] = g.out_off - (long long)g.h0 * g.nR + (r - g.r0);
     pstride[r] = g.nR;
+}
+
+// Region of every template (binary search over the regions' first-template indices).
+__global__ void k_template_regions(const int n_templates, const int n_regions, const RegionInfo* __restrict__ regs, int* __restrict__ region)
+{
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_templates) return;
+    int lo = 0, hi = n_regions;                 // largest g with regs[g].t0 <= t (every region owns at least one template)
+    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (regs[mid].t0 <= t) lo = mid; else hi = mid; }
+    region[t] = lo;
+}
+
+// Device-resident template offsets: non-decreasing, and the templates of every region cover exactly its reads. flags |= kFlagBadTemplates
+// otherwise (checked before the template epilogue reads through the offsets).
+__global__ void k_check_templates(const int n_templates, const long long* __restrict__ toff, const int* __restrict__ region,
+                                  const RegionInfo* __restrict__ regs, int* __restrict__ flags)
+{
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_templates) return;
+    const RegionInfo g = regs[region[t]];
+    const long long a = toff[t], b = toff[t + 1];
+    bool bad = b < a;
+    if (t == g.t0 && a != g.r0) bad = true;
+    if (t == g.t0 + g.nT - 1 && b != (long long)g.r0 + g.nR) bad = true;
+    if (bad) atomicOr(flags, kFlagBadTemplates);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1517,18 +1543,6 @@ k_align_reads_fast(const AlignParams p)
     }
 }
 
-// HaplotypeLikelihoodModel::evaluate(AlignedTemplate) (haplotype_likelihood_model.cpp:306-320): out[h][t] = sum over the
-// template's reads, accumulated in read order like std::accumulate.
-__global__ void k_template_sum(const double* __restrict__ lnl, const int H, const int R, const long long* __restrict__ toff, const int T,
-                               double* __restrict__ out)
-{
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (long long)H * T) return;
-    const int h = (int)(i / T), t = (int)(i % T);
-    double acc = 0.0;
-    for (long long r = toff[t]; r < toff[t + 1]; ++r) acc += lnl[(size_t)h * R + r];
-    out[i] = acc;
-}
 
 // N1 (SURVEY.md §8f): ConstantMixtureGenotypeLikelihoodModel::evaluate on the resident [H][R] matrix
 // (core/models/genotype/constant_mixture_genotype_likelihood_model.cpp:30-140): one block per genotype,
@@ -1580,6 +1594,33 @@ __global__ void k_epilogue(const int* __restrict__ best, int* __restrict__ statu
     if (b == kBestInf && status[i] == 0) status[i] = 1;
     // `out` may be another GPU's memory (a peer mapping, phmm_ipc_open): plain coalesced stores, nothing is read back
     out[i + hl * out_row_extra] = finish_likelihood(b, use_mapq != 0, rd.mapq[r], mapq_cap, mapq_trigger);
+}
+
+// Template epilogue: k_epilogue for the reads of one template and HaplotypeLikelihoodModel::evaluate(AlignedTemplate)
+// (haplotype_likelihood_model.cpp:306-320) in one pass — the per-read doubles never reach memory. Thread = (haplotype slot, template),
+// templates fastest: consecutive threads store consecutive outputs of a region's [nH][nT] matrix at tout_off.
+__global__ void k_template_epilogue(const int* __restrict__ best, int* __restrict__ status, const DevReads rd, const RegionInfo* __restrict__ regs,
+                                    const int Hmax, const int n_templates, const long long* __restrict__ toff, const int* __restrict__ tregion,
+                                    const int use_mapq, const int mapq_cap, const int mapq_trigger, const int* __restrict__ flags,
+                                    double* __restrict__ tout)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)Hmax * n_templates) return;
+    if (*flags & kFlagBadTemplates) return;        // offsets that k_check_templates rejected are not followed
+    int hl, t;
+    split_index(i, n_templates, &hl, &t);
+    const RegionInfo g = regs[tregion[t]];
+    if (hl >= g.nH) return;
+    const long long row = g.out_off + (long long)hl * g.nR - g.r0;     // pair_slot(rd, g.h0 + hl, r) == row + r
+    double acc = 0.0;
+    for (long long r = toff[t], end = toff[t + 1]; r < end; ++r) {
+        const long long s = row + r;
+        const int b = best[s];
+        if (b == kBestInf && status[s] == 0) status[s] = 1;
+        // the sum in read order from 0.0, like std::accumulate; __dadd_rn keeps the additions out of any fused multiply-add
+        acc = __dadd_rn(acc, finish_likelihood(b, use_mapq != 0, rd.mapq[r], mapq_cap, mapq_trigger));
+    }
+    tout[g.tout_off + (long long)hl * g.nT + (t - g.t0)] = acc;
 }
 
 } // namespace phmm
